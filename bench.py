@@ -13,8 +13,8 @@ decoded once per step.
   roofline  the dominant memory-bound kernel: the fused DC-shift + RCT + level-1 5/3 DWT
           (k_dwt53_fwd<3>): algorithmic bytes = samples x 8 B (one 4-byte read + one 4-byte
           write per sample per level, SURVEY.md 8d) / CUDA-event duration of that launch
-  cpu_baseline  the UNMODIFIED reference library (baseline/_ref/bin/libgrokj2k.so.1, built from
-          /root/reference by baseline/build_ref.sh): grk_compress() into a memory stream +
+  cpu_baseline  the UNMODIFIED reference library (oracle/_ref/grok/bin/libgrokj2k.so.1, built from
+          Grok's sources by oracle/build_grok.sh): grk_compress() into a memory stream +
           grk_decompress() from it (grok.cpp L1025 ff.; harness baseline/grk_ref_bench.cpp), same
           image, all host threads and one thread; the round-1 kernel composite (oracle/_ref) is
           kept as a second, labelled figure
@@ -227,7 +227,7 @@ def cpu_quota():
 
 
 # ------------------------------------------------------------------------------------------------
-# The reference itself: libgrokj2k's public API on memory streams (tests/grok_ref.py -> baseline/_ref)
+# The reference itself: libgrokj2k's public API on memory streams (tests/grok_ref.py -> oracle/_ref/grok)
 # ------------------------------------------------------------------------------------------------
 def grok_setup(img, w=W, h=H):
     import grok_ref as R
@@ -308,7 +308,7 @@ def run_reference(args, rank, world):
     img = make_image()
     st = grok_setup(img)
     if st is None:
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref (libgrokj2k built from /root/reference) is not in the tree"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/grok (libgrokj2k built from Grok's sources) is not in the tree"}))
         return
     grok_tune_threads(st)
     for _ in range(args.warmup):
@@ -334,7 +334,7 @@ def run_reference(args, rank, world):
             "decode_only": {"value": W * H / float(np.mean(decs)) / 1e6, "unit": "Mpixels/s", "ms": float(np.mean(decs)) * 1e3},
             "cpu_baseline": {"value": val, "unit": "Mpixels/s", "cores": st["threads"], "cpu_quota": cpu_quota(), "kind": "reference",
                              "sample": "whole image (64 of 64 tiles) per step: grk_compress() + grk_decompress() of the unmodified "
-                                       "libgrokj2k (baseline/_ref) on memory streams, TLM + PLT, %d threads" % st["threads"]},
+                                       "libgrokj2k (oracle/_ref/grok) on memory streams, TLM + PLT, %d threads" % st["threads"]},
             "e2e": {"value": val, "unit": "Mpixels/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
 
@@ -504,7 +504,12 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="config2", choices=["config2", "config4"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the device-resident round trip returned in its last step "
+                         "as DIR/<name>.npy (fixed seeded samples of the large arrays)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "config2"):
+        ap.error("--dump-outputs covers the config2 GPU workload only")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -572,6 +577,11 @@ def main():
     launches = lib.b2k_launch_count() - l0
     job.download(out)
     assert all(np.array_equal(a, b) for a, b in zip(out, planes)), "device-resident round trip is not lossless"
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        res = job.fetch_result()
+        dumped = sample_outputs(out, res)
+        res.free()
     pipe = None
     if world == 1 or bool(os.environ.get("B2K_BENCH_ALL_LEGS")):
         # extra: the same K round trips with the block-coder stage pipelined over 2 block ranges on 2 streams
@@ -630,10 +640,10 @@ def main():
             e2e_step()
         barrier()
         t0 = time.perf_counter()
-        for _ in range(max(3, args.steps // 2)):
+        for _ in range(args.steps):
             e2e_step()
         barrier()
-        dt_e2e32 = (time.perf_counter() - t0) / max(3, args.steps // 2)
+        dt_e2e32 = (time.perf_counter() - t0) / args.steps
         assert all(np.array_equal(a, b) for a, b in zip(out, planes)), "e2e (no host packing) round trip is not lossless"
         G.set_host_threads(-1)
 
@@ -649,10 +659,10 @@ def main():
             file_step()
         barrier()
         t0 = time.perf_counter()
-        for _ in range(max(3, args.steps // 2)):
+        for _ in range(args.steps):
             cs_len = file_step()
         barrier()
-        dt_file = (time.perf_counter() - t0) / max(3, args.steps // 2)
+        dt_file = (time.perf_counter() - t0) / args.steps
         assert all(np.array_equal(a, b) for a, b in zip(out, planes)), "codestream round trip is not lossless"
 
         # ---------------- same, 16-bit sample containers (b2k_encode16 / b2k_decode16) ----------------
@@ -721,7 +731,7 @@ def main():
 
         streamed(3 * depth + 3)           # warm-up: every worker's engine has built its job, the pinned result arenas exist
         barrier()
-        n_stream = max(16, args.steps)
+        n_stream = args.steps
         dt_stream = streamed(n_stream) / n_stream
         barrier()
         enc_stream.end()
@@ -809,7 +819,7 @@ def main():
                 cb = {"value": W * H / sec / 1e6, "unit": "Mpixels/s", "cores": gs["threads"], "cpu_quota": cpu_quota(),
                       "kind": "reference", "host": cpu_model(),
                       "sample": "whole image (64 of 64 tiles), best of 3 passes: grk_compress() + grk_decompress() of the unmodified "
-                                "libgrokj2k (baseline/_ref) on memory streams, TLM + PLT",
+                                "libgrokj2k (oracle/_ref/grok) on memory streams, TLM + PLT",
                       "encode_only_Mpix_s": W * H / info["enc_s"] / 1e6, "decode_only_Mpix_s": W * H / info["dec_s"] / 1e6, **info}
                 # one thread, on a 2048x2048 corner (4 of 64 tiles) so that it stays bounded
                 g1 = grok_setup(img, 2048, 2048)
@@ -824,7 +834,7 @@ def main():
                                                    "device_resident": value / cb["value"]}
             else:
                 line["cpu_baseline"] = {"value": None, "unit": "Mpixels/s", "cores": 0, "kind": "reference",
-                                        "sample": "baseline/_ref not built"}
+                                        "sample": "oracle/_ref/grok not built"}
             st = cpu_reference_setup(img)
             if st is not None:   # round 1's figure, kept for continuity: kernels only, no T2 / streams / scheduler
                 tune_reference_threads(st)
@@ -833,10 +843,35 @@ def main():
                                                 "sample": "whole image, best of 2: the reference's HT coder + forward DWT kernels and its "
                                                           "grk_bench_dwt_53 hook driven by oracle/ref_shim (no T2, no streams)", **info}
         print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
     eng.close()
+
+
+DUMP_SEED = 20261017
+DUMP_SAMPLES = 1 << 21
+
+
+def sample_outputs(planes, res):
+    """What the device-resident round trip hands back after its last step, cut to about 42 MB: the decoded image
+    and the coded bytes at fixed seeded positions, and the whole block table's lengths, bit planes and passes.
+    The coded bytes are sampled from the blocks laid end to end in enumeration order, so that the arena's
+    layout on the device does not matter.  float32 holds every decoded sample and byte exactly."""
+    rng = np.random.default_rng(DUMP_SEED)
+    pix = rng.integers(0, H * W, DUMP_SAMPLES)
+    lens = res.blocks["length"].astype(np.int64)
+    ends = np.cumsum(lens)
+    pos = rng.integers(0, int(ends[-1]), 2 * DUMP_SAMPLES)
+    blk = np.searchsorted(ends, pos, side="right")
+    at = res.blocks["offset"].astype(np.int64)[blk] + pos - (ends[blk] - lens[blk])
+    return {"decoded_sample": np.stack([p.reshape(-1)[pix] for p in planes]).astype(np.float32),
+            "coded_bytes_sample": res.bytes[at].astype(np.float32),
+            "block_table": np.stack([lens, res.blocks["numbps"], res.blocks["numpasses"]]).astype(np.float64)}
 
 
 # dram__bytes_read.sum + dram__bytes_write.sum of one k_dwt53_fwd<3> launch, from the committed `ncu --set full` capture

@@ -1,9 +1,9 @@
-"""ctypes binding of baseline/_ref/bin/libgrk_ref_bench.so: the UNMODIFIED reference library
-(libgrokj2k, built by baseline/build_ref.sh from /root/reference) driven through its public API --
+"""ctypes binding of oracle/_ref/grok/bin/libgrk_ref_bench.so: the UNMODIFIED reference library
+(libgrokj2k, built by oracle/build_grok.sh from the Grok source tree) driven through its public API --
 grk_compress() into a memory stream, grk_decompress() from one (baseline/grk_ref_bench.cpp).
 
 Test / measurement infrastructure only: tests/, bench.py's reference arm and cpu_baseline leg.
-`available()` is False when the reference was not built (no /root/reference at build time)."""
+`available()` is False when the reference was not built (no Grok source tree at build time)."""
 import ctypes as C
 import os
 import subprocess
@@ -11,9 +11,9 @@ import subprocess
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-# GROK_REF_FLAVOUR=patched selects the host built with baseline/patches/ applied (baseline/build_ref_patched.sh)
-FLAVOUR = "_ref_patched" if os.environ.get("GROK_REF_FLAVOUR") == "patched" else "_ref"
-BIN = os.path.join(ROOT, "baseline", FLAVOUR, "bin")
+# GROK_REF_FLAVOUR=patched selects the host built with baseline/patches/ applied (oracle/build_grok_patched.sh)
+FLAVOUR = "grok_patched" if os.environ.get("GROK_REF_FLAVOUR") == "patched" else "grok"
+BIN = os.path.join(ROOT, "oracle", "_ref", FLAVOUR, "bin")
 LIB = os.path.join(BIN, "libgrk_ref_bench.so")
 PLUGIN_DIR = os.path.join(ROOT, "grok_b200")     # holds libgrokj2k_plugin.so, the name the host's loader looks for
 
@@ -35,7 +35,7 @@ def lib():
     global _lib
     if _lib is None:
         if not available():
-            raise RuntimeError("baseline/_ref is not built (run baseline/build_ref.sh where /root/reference exists)")
+            raise RuntimeError("oracle/_ref/%s is not built (build() does it where the Grok source tree is)" % FLAVOUR)
         L = C.CDLL(LIB)
         L.grb_init.restype = C.c_int
         L.grb_init.argtypes = [C.c_uint32, C.c_char_p, C.c_int32]
@@ -143,6 +143,6 @@ def cli_env(extra=None):
 
 
 def run_cli(tool, args, env=None, timeout=600):
-    """Run baseline/_ref/bin/<tool> (grk_compress / grk_decompress / grk_dump); returns CompletedProcess."""
+    """Run oracle/_ref/grok/bin/<tool> (grk_compress / grk_decompress / grk_dump); returns CompletedProcess."""
     return subprocess.run([os.path.join(BIN, tool)] + list(args), env=cli_env(env), stdout=subprocess.PIPE,
                           stderr=subprocess.STDOUT, text=True, timeout=timeout)

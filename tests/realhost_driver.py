@@ -1,5 +1,5 @@
 """Runs in a SUBPROCESS of tests/test_realhost.py (a crash of the host library must not take pytest down):
-the real reference host -- stock (baseline/_ref) or patched (baseline/_ref_patched, GROK_REF_FLAVOUR=patched) --
+the real reference host -- stock (oracle/_ref/grok) or patched (oracle/_ref/grok_patched, GROK_REF_FLAVOUR=patched) --
 first on its own CPU path, then with grok_b200/libgrokj2k_plugin.so loaded through its own plugin loader
 (grk_initialize(plugin_path) + grk_plugin_init), and prints one JSON line comparing the two.
 

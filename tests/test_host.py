@@ -414,7 +414,7 @@ def test_bench_reference_arm_runs_to_completion_and_prints_its_json_line():
     line = json.loads(lines[0])
     assert line["impl"] == "reference"
     if "unavailable" in line:
-        assert not os.path.exists(os.path.join(root, "baseline", "_ref", "bin", "libgrk_ref_bench.so"))
+        assert not os.path.exists(os.path.join(root, "oracle", "_ref", "grok", "bin", "libgrk_ref_bench.so"))
         return
     assert line["unit"] == "Mpixels/s" and line["value"] > 0 and line["higher_is_better"] is True
     assert line["cpu_baseline"]["kind"] == "reference" and "grk_compress" in line["cpu_baseline"]["sample"]

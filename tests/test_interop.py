@@ -1,7 +1,9 @@
 """Interop parity gate against the REAL reference library (BASELINE.md 3.6).
 
-baseline/_ref/bin/libgrokj2k.so.1 is the unmodified GrokImageCompression/Grok built by baseline/build_ref.sh
-(SURVEY.md 8c recipe); tests/grok_ref.py drives its public API (grk_compress / grk_decompress on memory streams).
+The reference outputs are those of the unmodified GrokImageCompression/Grok (libgrokj2k built by
+oracle/build_grok.sh, driven through its public API by tests/grok_ref.py: grk_compress / grk_decompress on memory
+streams), kept in tests/golden/ by tests/golden/make_reference_golden.py: digests of its code streams and of its
+decoded images, its COM marker segments, and its decode itself where only a tolerance applies.
 What is pinned here, on the reference's own outputs:
 
 * reversible path: our codestream (b2k_codestream_write over oracle- or GPU-coded blocks) is BYTE-IDENTICAL to
@@ -13,23 +15,14 @@ What is pinned here, on the reference's own outputs:
   <= 8-bit irreversible images through its 16-bit fixed-point engine: a different algorithm; there the bar is
   the reference's own <= 2 codes, GrkPluginBatchMemoryTest.cpp L35-45).
 
-The CPU tests use the oracle as the block coder (no GPU), the `-m gpu` tests the CUDA engine.  Everything skips
-when baseline/_ref was not built (no reference tree at build time)."""
+The CPU tests use the oracle as the block coder (no GPU), the `-m gpu` tests the CUDA engine."""
 import numpy as np
 import pytest
 
 import grok_b200 as G
-import grok_ref as R
 import oracle_pipeline as P
+import reference_golden as RG
 from test_codestream import oracle_decode, oracle_encode
-
-pytestmark = pytest.mark.skipif(not R.available(), reason="baseline/_ref (the reference library) is not built")
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _grok():
-    R.init(4)
-    yield
 
 
 def strip_com(cs):
@@ -47,11 +40,17 @@ def strip_com(cs):
     return bytes(out) + cs[i:]
 
 
-def grok_compress(args, planes):
+def grok_compress(args, planes, R):
+    """grk_compress with TLM + PLT (`R`: tests/grok_ref.py; the golden data's generator calls this)"""
     cs, _ = R.compress(planes, args["prec"], tile=args.get("tile"), numres=args.get("numres", 6),
                        irreversible=args.get("irreversible", False), tlm=True, plt=True, cblk=args.get("cblk", (64, 64)),
                        precinct=args.get("grok_precinct"))
     return np.frombuffer(bytes(cs), np.uint8)
+
+
+def oracle_codestream(args, planes):
+    table, data, _ = oracle_encode(mk(args), planes)
+    return G.codestream_write(mk(args), table, data, G.CS_TLM | G.CS_PLT)
 
 
 def block_bytes(table, data, i):
@@ -96,12 +95,9 @@ def test_reversible_codestream_is_byte_identical_to_grok(args):
     planes = synth(args)
     table, data, _ = oracle_encode(cp, planes)
     ours = G.codestream_write(cp, table, data, G.CS_TLM | G.CS_PLT)
-    theirs = grok_compress(args, planes)
-    assert bytes(ours) == strip_com(theirs)
-    # Grok decodes ours exactly
-    dec, _, _ = R.decompress(ours, args["width"], args["height"], args["numcomps"])
-    for a, b in zip(dec, planes):
-        assert np.array_equal(a, b)
+    theirs = RG.grok_codestream(ours, args, 5)
+    # Grok decodes its stream, which is ours, exactly
+    assert RG.planes_sha(planes) == RG.grok_decoded(args, 5)
     # we decode Grok's exactly, block bytes equal
     cp2, blocks = G.codestream_parse(theirs)
     assert len(blocks) == len(table)
@@ -117,12 +113,10 @@ def test_precinct_spec_shorter_than_resolutions_matches_grok():
     (CodeStreamCompress.cpp L793-825).  The packet order then depends on the derived precinct grid."""
     args = dict(width=600, height=500, numcomps=3, prec=12, numres=5)
     planes = synth(args)
-    theirs, _ = R.compress(planes, 12, numres=5, tlm=True, plt=True, precinct=(128, 128))
-    theirs = np.frombuffer(bytes(theirs), np.uint8)
     cp = G.make_coding(precincts=[(max(128 >> k, 2),) * 2 for k in range(5)][::-1], **args)
     table, data, _ = oracle_encode(cp, planes)
     ours = G.codestream_write(cp, table, data, G.CS_TLM | G.CS_PLT)
-    assert bytes(ours) == strip_com(theirs)
+    RG.grok_codestream(ours, dict(args, grok_precinct=(128, 128)), 5)   # grk_compress -c [128,128]
 
 
 @pytest.mark.parametrize("args", IRREVERSIBLE)
@@ -131,16 +125,13 @@ def test_irreversible_blocks_are_byte_identical_to_grok(args):
     planes = synth(args)
     table, data, _ = oracle_encode(cp, planes)
     ours = G.codestream_write(cp, table, data, G.CS_TLM | G.CS_PLT)
-    theirs = grok_compress(args, planes)
+    theirs = RG.grok_codestream(ours, args, 5)
     cp2, blocks = G.codestream_parse(theirs)
     same = sum(int(np.array_equal(block_bytes(table, data, i), block_bytes(blocks, theirs, i))) for i in range(len(table)))
     assert same == len(table), "%d of %d irreversible code blocks equal Grok's" % (same, len(table))
-    assert bytes(ours) == strip_com(theirs)
     # decode: ours of theirs == Grok's of theirs, sample for sample (precision >= 9)
-    gd, _, _ = R.decompress(theirs, args["width"], args["height"], args["numcomps"])
     od = oracle_decode(cp2, blocks, theirs)
-    for a, b in zip(gd, od):
-        assert np.array_equal(a, b)
+    assert RG.planes_sha(od) == RG.grok_decoded(args, 5)
 
 
 def test_irreversible_8bit_decode_within_reference_tolerance():
@@ -150,11 +141,12 @@ def test_irreversible_8bit_decode_within_reference_tolerance():
     cp = mk(args)
     planes = synth(args)
     table, data, _ = oracle_encode(cp, planes)
-    theirs = grok_compress(args, planes)
+    theirs = RG.grok_codestream(G.codestream_write(cp, table, data, G.CS_TLM | G.CS_PLT), args, 5)
     cp2, blocks = G.codestream_parse(theirs)
     for i in range(len(table)):
         assert np.array_equal(block_bytes(table, data, i), block_bytes(blocks, theirs, i))
-    gd, _, _ = R.decompress(theirs, 320, 256, 3)
+    gd = RG.outputs()["decoded_8bit_irreversible_minus_source"] + np.stack(planes)      # Grok's decode
+    assert RG.planes_sha(gd) == RG.grok_decoded(args, 5)
     od = oracle_decode(cp2, blocks, theirs)
     for a, b in zip(gd, od):
         assert np.abs(a.astype(np.int64) - b).max() <= 2
@@ -168,20 +160,21 @@ def test_irreversible_8bit_decode_within_reference_tolerance():
 def test_gpu_codestream_is_byte_identical_to_grok_and_decodes_it(engine, args):
     cp = mk(args)
     planes = synth(args, seed=9)
-    theirs = grok_compress(args, planes)
     ours = engine.encode_codestream(cp, planes, flags=G.CS_TLM | G.CS_PLT)
-    assert bytes(ours) == strip_com(theirs), "GPU codestream differs from grk_compress's"
-    # Grok decodes the GPU's stream; the GPU decodes Grok's stream; both equal Grok decoding its own
-    w, h, n = args["width"], args["height"], args["numcomps"]
-    g_of_ours, _, _ = R.decompress(ours, w, h, n)
-    g_of_theirs, _, _ = R.decompress(theirs, w, h, n)
+    theirs = RG.grok_codestream(ours, args, 9)
+    # the GPU decodes Grok's stream (which Grok decodes as its own: it is the GPU's) to what Grok gave back
     _, ours_of_theirs = engine.decode_codestream(theirs)
-    for a, b, c, src in zip(g_of_ours, g_of_theirs, ours_of_theirs, planes):
-        assert np.array_equal(a, b)
-        if args.get("irreversible"):
+    if args.get("irreversible"):
+        # Grok's decode of >= 9-bit 9/7 streams is the oracle's, sample for sample (test_irreversible_blocks_are_...)
+        cp2, blocks = G.codestream_parse(theirs)
+        g_of_theirs = oracle_decode(cp2, blocks, theirs)
+        assert RG.planes_sha(g_of_theirs) == RG.grok_decoded(args, 9)
+        for b, c in zip(g_of_theirs, ours_of_theirs):
             assert np.abs(c.astype(np.int64) - b).max() <= 1      # device inverse 9/7 vs Grok's host inverse
-        else:
-            assert np.array_equal(c, src) and np.array_equal(b, src)
+    else:
+        assert RG.planes_sha(planes) == RG.grok_decoded(args, 9)
+        for c, src in zip(ours_of_theirs, planes):
+            assert np.array_equal(c, src)
 
 
 @pytest.mark.gpu
@@ -190,9 +183,8 @@ def test_gpu_config2_tiles_match_grok_at_full_tile_size(engine):
     args = dict(width=2048, height=2048, numcomps=3, prec=12, tile=(1024, 1024))
     cp = mk(args)
     planes = P.synthetic_image(2048, 2048, 3, 12, seed=20260924)
-    theirs = grok_compress(args, planes)
     ours = engine.encode_codestream(cp, planes, flags=G.CS_TLM | G.CS_PLT)
-    assert bytes(ours) == strip_com(theirs)
+    theirs = RG.grok_codestream(ours, args, 20260924)
     _, rec = engine.decode_codestream(theirs)
     for a, b in zip(rec, planes):
         assert np.array_equal(a, b)
@@ -201,6 +193,10 @@ def test_gpu_config2_tiles_match_grok_at_full_tile_size(engine):
 # ------------------------------------------------------------------------------------------------------
 # BASELINE.json's configurations at the sizes they name (VERDICT r1 item 9), against the real library
 # ------------------------------------------------------------------------------------------------------
+CONFIG3 = dict(width=8192, height=8192, numcomps=3, prec=12, numres=6, irreversible=True)
+CONFIG4 = dict(width=16384, height=16384, numcomps=4, prec=16, numres=6, tile=(1024, 1024), mct=1)
+
+
 @pytest.mark.gpu
 def test_config3_full_size_single_tile_irreversible_matches_grok(engine):
     """configs[2]: 8192x8192x3 12-bit, ONE tile, 9/7 + ICT, 5 levels (6 resolutions), 64x64 blocks.  The GPU's code
@@ -208,15 +204,15 @@ def test_config3_full_size_single_tile_irreversible_matches_grok(engine):
     GPU's decode of it must agree with Grok's own to within one code (device inverse 9/7 vs host; the reference's bar is
     <= 2, GrkPluginBatchMemoryTest.cpp L35-45) and sit > 50 dB from the source (GrkPluginMemoryTest.cpp L39-52)."""
     w = h = 8192
-    cp = G.make_coding(w, h, 3, 12, numres=6, irreversible=True)
+    cp = mk(CONFIG3)
     planes = P.synthetic_image(w, h, 3, 12, seed=20260925)
-    R.init(0)
-    theirs, _ = R.compress(planes, 12, numres=6, irreversible=True, tlm=True, plt=True)
-    theirs = np.frombuffer(bytes(theirs), np.uint8)
     ours = engine.encode_codestream(cp, planes, flags=G.CS_TLM | G.CS_PLT)
-    assert bytes(ours) == strip_com(theirs)
+    theirs = RG.grok_codestream(ours, CONFIG3, 20260925)
     _, rec = engine.decode_codestream(theirs)
-    gd, _, _ = R.decompress(theirs, w, h, 3)
+    # Grok's decode of a 12-bit 9/7 stream is the oracle's, sample for sample
+    cp2, blocks = G.codestream_parse(theirs)
+    gd = oracle_decode(cp2, blocks, theirs)
+    assert RG.planes_sha(gd) == RG.grok_decoded(CONFIG3, 20260925)
     for a, b, s in zip(rec, gd, planes):
         assert np.abs(a.astype(np.int64) - b).max() <= 1
         err = (a.astype(np.float64) - s)
@@ -229,16 +225,13 @@ def test_config4_full_size_sharded_tiles_match_grok(engine):
     as two shards (tile t -> shard t % 2, what two ranks would do), merged with b2k_result_merge and written as ONE
     code stream: byte-identical to grk_compress's, and the decode of Grok's stream gives the source back."""
     w = h = 16384
-    cp = G.make_coding(w, h, 4, 16, numres=6, tile=(1024, 1024), mct=1)
+    cp = mk(CONFIG4)
     base = P.synthetic_image(1024, 1024, 4, 16, seed=20260926)
     planes = [np.empty((h, w), np.int32) for _ in range(4)]
     for t in range(256):
         ty, tx = divmod(t, 16)
         for c in range(4):
             planes[c][ty * 1024:(ty + 1) * 1024, tx * 1024:(tx + 1) * 1024] = (base[c] + 257 * t) & 0xFFFF
-    R.init(0)
-    theirs, _ = R.compress(planes, 16, tile=(1024, 1024), numres=6, tlm=True, plt=True, mct=1)
-    theirs = np.frombuffer(bytes(theirs), np.uint8)
     shards = []
     for rem in (0, 1):
         r = engine.encode(cp, planes, tile_mod=2, tile_rem=rem)
@@ -247,7 +240,7 @@ def test_config4_full_size_sharded_tiles_match_grok(engine):
     merged = G.merge_shards(cp, shards)
     ours = G.codestream_write(cp, merged.blocks, merged.bytes, G.CS_TLM | G.CS_PLT, num_tiles=256)
     merged.free()
-    assert bytes(ours) == strip_com(theirs)
+    theirs = RG.grok_codestream(ours, CONFIG4, 20260926)
     del ours, shards
     _, rec = engine.decode_codestream(theirs)
     for a, b in zip(rec, planes):
@@ -283,30 +276,31 @@ WINDOW_CASES = [
 ]
 
 
+def window_args(args, window, reduce):
+    return dict(args, window=window, reduce=reduce)
+
+
 @pytest.mark.parametrize("args,window,reduce", WINDOW_CASES)
 def test_window_and_reduce_parse_matches_grok(args, window, reduce):
     """The virtual coding decodes (on the oracle) to exactly what Grok delivers for the same window / reduce factor:
     grk_decompress at `reduce` gives the reference for the resolution, the window is a crop of it."""
-    cp = mk(args)
     planes = synth(args, seed=12)
-    theirs = grok_compress(args, planes)
-    w, h, n = args["width"], args["height"], args["numcomps"]
-    rw, rh = -(-w >> reduce), -(-h >> reduce)
-    ref, _, _ = R.decompress(theirs, rw, rh, n, reduce=reduce)                # Grok's own reduced decode of the whole image
-    if reduce == 0 and not args.get("irreversible"):
-        for a, b in zip(ref, planes):
-            assert np.array_equal(a, b)
-    vcp, blocks = _parse_window(theirs, window, reduce)
-    rec = oracle_decode(vcp, blocks, theirs)
+    theirs = RG.grok_codestream(oracle_codestream(args, planes), args, 12)
+    w, h = args["width"], args["height"]
+    # Grok's own reduced decode of the whole image, cropped to the window
+    ref = RG.grok_decoded(window_args(args, window, reduce), 12, "window")
     sh = (1 << reduce) - 1
     full_win = (0, 0, w, h) if window is None else window
     x0, y0, x1, y1 = [(v + sh) >> reduce for v in full_win]
+    if reduce == 0 and not args.get("irreversible"):
+        assert RG.planes_sha([p[y0:y1, x0:x1] for p in planes]) == ref
+    vcp, blocks = _parse_window(theirs, window, reduce)
+    rec = oracle_decode(vcp, blocks, theirs)
     assert vcp.x0 <= x0 and vcp.y0 <= y0 and vcp.x1 >= x1 and vcp.y1 >= y1
     if window is not None:       # tile-granular: at most the touched tiles are decoded
         tw, th = args.get("tile", (w, h))
         assert (vcp.x1 - vcp.x0) <= ((-(-window[2] // tw) - window[0] // tw) * tw + sh) >> reduce
-    for a, b in zip(rec, ref):
-        assert np.array_equal(a[y0 - vcp.y0:y1 - vcp.y0, x0 - vcp.x0:x1 - vcp.x0], b[y0:y1, x0:x1])
+    assert RG.planes_sha([a[y0 - vcp.y0:y1 - vcp.y0, x0 - vcp.x0:x1 - vcp.x0] for a in rec]) == ref
 
 
 @pytest.mark.parametrize("irreversible", [False, True])
@@ -316,7 +310,7 @@ def test_window_parse_keeps_exactly_the_blocks_a_window_can_depend_on(irreversib
     decode, and most of the touched tiles' coded bytes are not needed."""
     args = dict(width=768, height=640, numcomps=1, prec=12, tile=(512, 512), numres=6, irreversible=irreversible)
     planes = synth(args, seed=21)
-    theirs = grok_compress(args, planes)
+    theirs = RG.grok_codestream(oracle_codestream(args, planes), args, 21)
     fcp, fblocks = G.codestream_parse(theirs)
     full = oracle_decode(fcp, fblocks, theirs)
     rng = np.random.default_rng(7)
@@ -338,14 +332,9 @@ def test_window_parse_keeps_exactly_the_blocks_a_window_can_depend_on(irreversib
 @pytest.mark.parametrize("args,window,reduce", WINDOW_CASES)
 def test_gpu_window_and_reduce_decode_matches_grok(engine, args, window, reduce):
     planes = synth(args, seed=12)
-    theirs = grok_compress(args, planes)
-    w, h, n = args["width"], args["height"], args["numcomps"]
-    ref, _, _ = R.decompress(theirs, -(-w >> reduce), -(-h >> reduce), n, reduce=reduce)
+    theirs = RG.grok_codestream(engine.encode_codestream(mk(args), planes, flags=G.CS_TLM | G.CS_PLT), args, 12)
     _, got = engine.decode_window(theirs, window, reduce)
-    sh = (1 << reduce) - 1
-    x0, y0, x1, y1 = [(v + sh) >> reduce for v in ((0, 0, w, h) if window is None else window)]
-    for a, b in zip(got, ref):
-        assert np.array_equal(a, b[y0:y1, x0:x1])
+    assert RG.planes_sha(got) == RG.grok_decoded(window_args(args, window, reduce), 12, "window")
 
 
 @pytest.mark.gpu

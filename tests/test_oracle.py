@@ -1,6 +1,7 @@
 """CPU tests (-m "not gpu"): the oracle against the committed golden vectors (made from the
-reference's own kernels by tests/golden/make_golden.py), against oracle/_ref live when that
-library is present, and the reference's own round-trip properties (SURVEY.md section 4)."""
+reference's own kernels by tests/golden/make_golden.py), against the reference kernels' outputs
+for seeded random inputs (digests by tests/golden/make_reference_golden.py), and the reference's own
+round-trip properties (SURVEY.md section 4)."""
 import os
 
 import numpy as np
@@ -8,6 +9,7 @@ import pytest
 
 import oracle_lib as O
 import oracle_pipeline as P
+import reference_golden as RG
 import grok_b200 as G
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -54,46 +56,57 @@ def test_dwt_forward_matches_reference_golden(dwt_gold):
         assert np.array_equal(f.view(np.int32), dwt_gold["dwt97_%d" % i].view(np.int32)), i  # bit exact
 
 
-@pytest.mark.skipif(O.ref() is None, reason="oracle/_ref not built (no reference tree here)")
-def test_oracle_vs_reference_live():
+def live_cases():
+    """The seeded code blocks and tiles of test_oracle_vs_reference_live (also what the reference was given)."""
     rng = np.random.default_rng(11)
-    L, R = O.lib(), O.ref()
+    blocks, tiles = [], []
     for _ in range(60):
         w = int(rng.choice([1, 2, 3, 5, 8, 31, 32, 33, 64, 100]))
         h = int(rng.choice([1, 2, 3, 4, 17, 32, 40]))
         kmax = int(rng.integers(1, 20))
         lim = (1 << kmax) - 1
         c = np.clip((rng.standard_normal((h, w)) * rng.choice([0, 2, 40, lim])).astype(np.int64), -lim, lim)
-        sm = O.to_sgnmag(c, kmax)
-        ours = O.ht_encode(sm, kmax)
-        for v in (0, 1, 2):
-            theirs = O.ref_ht_encode(sm, kmax, v)
-            if theirs is not None:
-                assert np.array_equal(ours, theirs)
-        rc, d = O.ht_decode(ours, kmax, w, h)
-        for v in (0, 1, 2):
-            rc2, d2 = O.ref_ht_decode(ours, kmax, w, h, v)
-            if rc2 != -2:
-                assert rc == 0 and rc2 == 0 and np.array_equal(d, d2)
+        blocks.append((O.to_sgnmag(c, kmax), kmax))
     for _ in range(30):
         x0, y0 = int(rng.integers(0, 9)), int(rng.integers(0, 9))
         w, h = int(rng.integers(1, 90)), int(rng.integers(1, 70))
         numres = int(rng.integers(1, 7))
-        stride = ((w + 15) // 16) * 16 + 16
-        a = O.aligned_zeros((h + 2, stride), np.int32)
-        a[:h, :w] = rng.integers(-4096, 4096, (h, w))
-        b = O.aligned_zeros((h + 2, stride), np.int32)
-        b[:] = a
-        L.orc_dwt53_fwd_2d(a, stride, x0, y0, x0 + w, y0 + h, numres)
-        R.ref_dwt53_fwd_2d(b, stride, x0, y0, x0 + w, y0 + h, numres, 0)
-        assert np.array_equal(a[:h, :w], b[:h, :w])
-        f = O.aligned_zeros((h + 2, stride), np.float32)
-        f[:h, :w] = rng.integers(-4096, 4096, (h, w)).astype(np.float32)
-        g = O.aligned_zeros((h + 2, stride), np.float32)
-        g[:] = f
-        L.orc_dwt97_fwd_2d(f, stride, x0, y0, x0 + w, y0 + h, numres)
-        R.ref_dwt97_fwd_2d(g, stride, x0, y0, x0 + w, y0 + h, numres, 0.0, 0)
-        assert np.array_equal(f[:h, :w].view(np.int32), g[:h, :w].view(np.int32))
+        src = rng.integers(-4096, 4096, (h, w))
+        fsrc = rng.integers(-4096, 4096, (h, w)).astype(np.float32)
+        tiles.append(((x0, y0, w, h, numres), src, fsrc))
+    return blocks, tiles
+
+
+def dwt_fwd_aligned(fn, src, x0, y0, numres, *extra):
+    """Forward DWT of `src` in place in a 64-byte aligned, padded tile buffer (the reference's SIMD kernels
+    need one); returns the transformed (h, w) window."""
+    h, w = src.shape
+    stride = ((w + 15) // 16) * 16 + 16
+    a = O.aligned_zeros((h + 2, stride), src.dtype)
+    a[:h, :w] = src
+    fn(a, stride, x0, y0, x0 + w, y0 + h, numres, *extra)
+    return a[:h, :w]
+
+
+def test_oracle_vs_reference_live():
+    """HT encode / decode and both forward DWTs of seeded random blocks and tiles equal what the reference's own
+    kernels (every SIMD variant they have) computed from the same inputs."""
+    want = RG.digests()["oracle"]
+    blocks, tiles = live_cases()
+    L = O.lib()
+    for i, (sm, kmax) in enumerate(blocks):
+        h, w = sm.shape
+        ours = O.ht_encode(sm, kmax)
+        enc = [d for d in want["ht_encode"][i] if d is not None]
+        assert enc and all(RG.sha(ours) == d for d in enc), i
+        rc, d = O.ht_decode(ours, kmax, w, h)
+        for rc2, d2 in want["ht_decode"][i]:
+            if rc2 != -2:
+                assert rc == 0 and rc2 == 0 and RG.sha(d) == d2, i
+    for i, ((x0, y0, w, h, numres), src, fsrc) in enumerate(tiles):
+        a = dwt_fwd_aligned(L.orc_dwt53_fwd_2d, src.astype(np.int32), x0, y0, numres)
+        f = dwt_fwd_aligned(L.orc_dwt97_fwd_2d, fsrc, x0, y0, numres)
+        assert [RG.sha(a), RG.sha(f.view(np.int32))] == want["dwt"][i], i
 
 
 def test_reversible_exponents_known_answer():
@@ -198,10 +211,10 @@ def test_ht_refinement_passes_match_reference_golden():
     assert seen == {(2, 0), (2, 1), (3, 0), (3, 1)}
 
 
-@pytest.mark.skipif(O.ref() is None, reason="oracle/_ref not built (no reference tree here)")
-def test_ht_refinement_vs_reference_live():
+def refine_cases():
+    """The seeded blocks of test_ht_refinement_vs_reference_live: (w, h, missing MSBs, sign-magnitude samples)."""
     rng = np.random.default_rng(77)
-    for trial in range(60):
+    for _ in range(60):
         w, h = int(rng.integers(1, 65)), int(rng.integers(1, 65))
         M = int(rng.integers(8, 28))
         p = 30 - M
@@ -210,16 +223,28 @@ def test_ht_refinement_vs_reference_live():
         mag = np.minimum(mag, (1 << (31 - (p - 1))) - 1)
         v = (mag << np.uint64(p - 1)).astype(np.uint32)
         sm = np.where(v != 0, v | (rng.integers(0, 2, (h, w)).astype(np.uint32) << 31), 0).astype(np.uint32)
-        cup = O.ht_encode(sm, M)
+        yield w, h, M, sm
+
+
+def refine_stream(sm, M, npass, causal):
+    """cleanup + refinement segments of one block, and the refinement segment's length"""
+    seg = O.ht_encode_refine(sm, M, npass, causal)
+    return np.concatenate([O.ht_encode(sm, M), seg]), len(seg)
+
+
+def test_ht_refinement_vs_reference_live():
+    """2- and 3-pass streams of seeded blocks: the oracle decodes them to what the reference's decoder made of the
+    same streams."""
+    want = RG.digests()["refine"]
+    for trial, (w, h, M, sm) in enumerate(refine_cases()):
+        p = 30 - M
         for npass in (2, 3):
             for causal in (False, True):
-                seg = O.ht_encode_refine(sm, M, npass, causal)
-                data = np.concatenate([cup, seg])
-                rc1, a = O.ht_decode_passes(data, len(seg), npass, M, w, h, causal=causal)
-                rc2, b = O.ref_ht_decode(data, M, w, h, variant=-1, num_passes=npass, len2=len(seg), causal=causal)
-                assert rc1 == 0 and rc2 == 0 and np.array_equal(a, b), (trial, npass, causal)
+                data, len2 = refine_stream(sm, M, npass, causal)
+                rc1, a = O.ht_decode_passes(data, len2, npass, M, w, h, causal=causal)
+                assert rc1 == 0 and [RG.sha(data), RG.sha(a)] == want[trial]["%d%d" % (npass, causal)], (trial, npass, causal)
                 if npass == 3:   # cleanup-significant samples are exact down to plane p-1
                     m = sm & 0x7FFFFFFF
                     cs = (m >> p) != 0
-                    want = ((m >> (p - 1)) << (p - 1)) | (1 << (p - 2)) | (sm & 0x80000000)
-                    assert np.array_equal(a[cs], want[cs])
+                    want_a = ((m >> (p - 1)) << (p - 1)) | (1 << (p - 2)) | (sm & 0x80000000)
+                    assert np.array_equal(a[cs], want_a[cs])

@@ -2,8 +2,8 @@
 loader enabled -- dlopens grok_b200/libgrokj2k_plugin.so through its own minpf loader, resolves minpf_post_load_plugin /
 plugin_init / gpup_encode_mem / plugin_decompress by name and routes grk_compress() / grk_decompress() through them.
 
-* stock host (baseline/_ref, unmodified sources): single-tile images (the stock contract);
-* patched host (baseline/_ref_patched = sources + baseline/patches/0001-multi-tile-plugin-encode-decode.patch):
+* stock host (oracle/_ref/grok, unmodified sources): single-tile images (the stock contract);
+* patched host (oracle/_ref/grok_patched = sources + baseline/patches/0001-multi-tile-plugin-encode-decode.patch):
   multi-tile images through gpup_encode_mem_tiles / plugin_decompress_codestream.
 The assertion is the strongest one available: the code stream the host writes with the plugin's code blocks is
 byte-identical to the one it writes on its own CPU path, and the pixels it hands back are identical.
@@ -20,8 +20,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 
 
+HOST_DIR = {"_ref": "grok", "_ref_patched": "grok_patched"}     # flavour -> oracle/_ref/<dir> (oracle/build_grok*.sh)
+
+
 def built(flavour):
-    return os.path.exists(os.path.join(ROOT, "baseline", flavour, "bin", "libgrk_ref_bench.so"))
+    return os.path.exists(os.path.join(ROOT, "oracle", "_ref", HOST_DIR[flavour], "bin", "libgrk_ref_bench.so"))
 
 
 def run(case, flavour):
@@ -42,7 +45,7 @@ def test_host_loads_the_plugin_and_falls_back_without_a_device(flavour):
     """CPU box: the loader finds the library, every symbol resolves, plugin_init says "no device", the host carries on
     on its own path (grok.cpp L1344-1370) -- and nothing crashes on the way."""
     if not built(flavour):
-        pytest.skip("baseline/%s not built" % flavour)
+        pytest.skip("oracle/_ref/%s not built" % HOST_DIR[flavour])
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present: covered by the gpu tests")
@@ -66,7 +69,7 @@ STOCK_CASES = [
 @pytest.mark.parametrize("case", STOCK_CASES)
 def test_stock_host_compresses_and_decompresses_through_the_plugin(case):
     if not built("_ref"):
-        pytest.skip("baseline/_ref not built")
+        pytest.skip("oracle/_ref/grok not built")
     r = run(case, "_ref")
     assert r["plugin_loaded"], "the host did not load / initialise the plugin"
     assert r["plugin"]["enc_accelerated"] == 1, "grk_compress did not take the plugin route"
@@ -90,7 +93,7 @@ PATCHED_CASES = [
 @pytest.mark.parametrize("case", PATCHED_CASES)
 def test_patched_host_multi_tile_through_the_plugin(case):
     if not built("_ref_patched"):
-        pytest.skip("baseline/_ref_patched not built")
+        pytest.skip("oracle/_ref/grok_patched not built")
     r = run(case, "_ref_patched")
     assert r["plugin_loaded"]
     assert r["plugin"]["enc_accelerated"] == 1, "multi-tile grk_compress did not take gpup_encode_mem_tiles"
@@ -105,7 +108,7 @@ def test_patched_host_multi_tile_through_the_plugin(case):
 @pytest.mark.gpu
 def test_patched_host_still_serves_single_tile_through_the_stock_symbols():
     if not built("_ref_patched"):
-        pytest.skip("baseline/_ref_patched not built")
+        pytest.skip("oracle/_ref/grok_patched not built")
     r = run(dict(width=512, height=512, numcomps=1, prec=8), "_ref_patched")
     assert r["plugin_loaded"] and r["plugin"]["enc_accelerated"] == 1 and r["plugin"]["codestream_identical"]
     assert r["plugin"]["dec_accelerated"] == 1 and r["plugin"]["decode_identical"]
@@ -127,7 +130,7 @@ def test_stock_host_batch_interfaces_through_the_plugin(case):
     and every code stream equals the one grk_compress() writes on its own; code streams go in through the pull callback,
     the frames that come back equal grk_decompress()'s."""
     if not built("_ref"):
-        pytest.skip("baseline/_ref not built")
+        pytest.skip("oracle/_ref/grok not built")
     r = run(case, "_ref")
     assert r["declined_without_plugin"] == 1
     assert r["plugin_loaded"]
@@ -143,7 +146,7 @@ def test_stock_host_batch_interfaces_through_the_plugin(case):
 def test_batch_interfaces_decline_without_a_device():
     """no GPU: plugin_init fails, so both batch begins answer 1 and the caller stays on the CPU (grok.h)"""
     if not built("_ref"):
-        pytest.skip("baseline/_ref not built")
+        pytest.skip("oracle/_ref/grok not built")
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present: covered by the gpu tests")
