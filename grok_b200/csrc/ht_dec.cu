@@ -1,24 +1,23 @@
 /*
- * grok_b200/csrc/ht_dec.cu -- HTJ2K (ITU-T T.814) cleanup-pass block DECODER for sm_100a, one
- * warp per code block, fused with the T1 post-processing (dequantisation into the Mallat buffer).
+ * grok_b200/csrc/ht_dec.cu -- HTJ2K (ITU-T T.814) cleanup-pass block DECODER for sm_100a, fused with
+ * the T1 post-processing (dequantisation into the Mallat buffer).
  *
  * Replaces (reference, CPU): T1OJPH::decompress            t1/part15/CoderOJPH.cpp L212-262
  *                            ojph_decode_codeblock32        t1/part15/coding/ojph_block_decoder32.cpp L742-1317
  *                            ShiftOJPHFilter/ScaleOJPHFilter t1/part15/PostDecodeFiltersOJPH.h L48-66, L100-119
- * The cleanup pass is all Grok's own encoder ever emits (CoderOJPH.cpp L200-205) and is the fast
- * path (k_ht_decode_vlc + k_ht_decode_magsgn).  Blocks of foreign streams that carry SigProp /
- * MagRef refinement (ojph_block_decoder32.cpp L1318-1616) leave the cleanup kernels as raw
- * sign-magnitude words and are finished by k_ht_decode_refine, which also dequantises them.
- *
- * Per quad row:  (a) the MEL + CxtVLC + UVLC symbols of the row are decoded serially --
- * context-adaptive variable-length codes have no parallel parse -- by every lane redundantly
- * (uniform code, uniform loads) into a shared-memory record per quad;  (b) the MagSgn stream is
- * parsed by the whole warp: the per-sample bit counts follow from the records, a warp prefix
- * sum gives every lane its bit offset into an un-stuffed shared-memory bit ring that is refilled
- * 32 bytes at a time (one byte per lane, stuffing resolved with one ballot since on the decode
- * side a byte's width only depends on its predecessor's VALUE).
+ * The cleanup pass is all Grok's own encoder ever emits (CoderOJPH.cpp L200-205).  It is decoded in two
+ * launches:
+ *  (a) k_ht_decode_vlc, one THREAD per code block: the MEL + CxtVLC + U-VLC symbols, which have no
+ *      parallel parse, are decoded serially into one record per quad in global scratch;
+ *  (b) k_ht_decode_magsgn, one WARP per code block: per quad row the per-sample bit counts follow from
+ *      the records, a warp prefix sum gives every lane its bit offset into an un-stuffed shared-memory
+ *      bit ring that is refilled 256 bytes at a time (8 bytes per lane, stuffing resolved with one
+ *      ballot since on the decode side a byte's width only depends on its predecessor's VALUE), and the
+ *      lanes dequantise their quads straight into the Mallat buffer.
+ * Blocks of foreign streams that carry SigProp / MagRef refinement (ojph_block_decoder32.cpp
+ * L1318-1616) leave (b) as raw sign-magnitude words and are finished by k_ht_decode_refine, which also
+ * dequantises them.
  */
-#include <cstdlib>
 #include "b2k_internal.h"
 #define HT_TABLE_QUAL static __device__ const
 #include "ht_tables.h"
@@ -27,98 +26,8 @@ namespace {
 
 constexpr int MS_RING_WORDS = 256;
 
-__device__ __forceinline__ unsigned lanemask_lt_d()
-{
-  unsigned m;
-  asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
-  return m;
-}
 __device__ __forceinline__ int mel_exp_d(int k) { return (int)((0x58da489200ull >> (3 * k)) & 7ull); }
 
-/* ---- uniform (all lanes identical) serial readers ------------------------------------------ */
-struct MelR
-{ /* mel_read / mel_decode, ojph_block_decoder32.cpp L92-206 */
-  const uint8_t* d;
-  int size, pos, bits, unstuff, k, run, have;
-  uint32_t tmp;
-};
-__device__ __forceinline__ int mel_bit(MelR& m)
-{
-  if(m.bits == 0)
-  {
-    uint32_t v = 0xFF;
-    if(m.pos < m.size)
-    {
-      v = __ldg(m.d + m.pos);
-      if(m.pos == m.size - 1)
-        v |= 0xF;
-      m.pos++;
-    }
-    m.bits = 8 - m.unstuff;
-    m.tmp = v;
-    m.unstuff = (v == 0xFF);
-  }
-  m.bits--;
-  return (int)((m.tmp >> m.bits) & 1u);
-}
-__device__ __forceinline__ int mel_symbol(MelR& m)
-{
-  if(!m.have)
-  {
-    const int ev = mel_exp_d(m.k);
-    if(mel_bit(m))
-    {
-      m.run = 1 << ev;
-      m.have = 1;
-      m.k = min(12, m.k + 1);
-    }
-    else
-    {
-      int r = 0;
-      for(int i = 0; i < ev; ++i)
-        r = (r << 1) | mel_bit(m);
-      m.run = r;
-      m.have = 2;
-      m.k = max(0, m.k - 1);
-    }
-  }
-  if(m.run > 0)
-  {
-    m.run--;
-    if(m.run == 0 && m.have == 1)
-      m.have = 0;
-    return 0;
-  }
-  m.have = 0;
-  return 1;
-}
-
-struct VlcR
-{ /* rev_read / rev_init, L296-395 */
-  const uint8_t* d;
-  int pos, lo, bits, unstuff;
-  uint64_t tmp;
-};
-__device__ __forceinline__ uint32_t vlc_peek(VlcR& v)
-{
-  while(v.bits <= 56)
-  {
-    uint32_t b = 0;
-    if(v.pos >= v.lo)
-      b = __ldg(v.d + v.pos);
-    v.pos--;
-    const int nb = 8 - ((v.unstuff && ((b & 0x7F) == 0x7F)) ? 1 : 0);
-    v.tmp |= (uint64_t)b << v.bits;
-    v.bits += nb;
-    v.unstuff = b > 0x8F;
-  }
-  return (uint32_t)v.tmp;
-}
-__device__ __forceinline__ void vlc_skip(VlcR& v, int n)
-{
-  v.tmp >>= n;
-  v.bits -= n;
-}
 __device__ __forceinline__ int uvlc_prefix(uint32_t bits, int& len)
 {
   if(bits & 1) { len = 1; return 1; }
@@ -154,23 +63,6 @@ __device__ __forceinline__ T warp_excl_scan_d(T v, int lane, T& total)
  * interleaved word by word (entry k of a block sits at rec_off + 32 k): the 32 lanes of this kernel
  * -- 32 different blocks at the same quad -- store 128 contiguous bytes instead of 32 scattered words.
  * =========================================================================================== */
-/* refill so that at least 32 un-stuffed bits are buffered: one quad pair consumes at most
-   7+7 (CxtVLC) + 3+3+5+5 (UVLC) + 1 = 31 bits, so the parse of a pair needs no further checks */
-__device__ __forceinline__ void vlc_fill32(VlcR& v)
-{
-  while(v.bits < 32)
-  {
-    uint32_t b = 0;
-    if(v.pos >= v.lo)
-      b = __ldg(v.d + v.pos);
-    v.pos--;
-    const int nb = 8 - ((v.unstuff && ((b & 0x7F) == 0x7F)) ? 1 : 0);
-    v.tmp |= (uint64_t)b << v.bits;
-    v.bits += nb;
-    v.unstuff = b > 0x8F;
-  }
-}
-__device__ __forceinline__ uint32_t vlc_head(const VlcR& v) { return (uint32_t)v.tmp; }
 
 /* ---- phase A readers: the serial parse is latency-bound, so its byte streams must not put a global load into the
  * dependency chain for every byte.  Both streams are read through an aligned 8-byte register window with the NEXT
@@ -316,225 +208,18 @@ __device__ __forceinline__ int melf_symbol(MelFast& m)
   return 1;
 }
 
-/* significance of the previous / current quad row's bottom samples, one bit per quad.
-   WIDE = false: blocks at most 64 samples wide (32 quads) -> plain registers. */
-template <bool WIDE>
-struct SigRows
-{
-  uint32_t pbl[WIDE ? 16 : 1], pbr[WIDE ? 16 : 1], cbl[WIDE ? 16 : 1], cbr[WIDE ? 16 : 1];
-  __device__ __forceinline__ void clear()
-  {
-#pragma unroll
-    for(int i = 0; i < (WIDE ? 16 : 1); ++i)
-      pbl[i] = pbr[i] = cbl[i] = cbr[i] = 0;
-  }
-  __device__ __forceinline__ int prev_bl(int q) const { return (int)((pbl[WIDE ? (q >> 5) : 0] >> (q & 31)) & 1u); }
-  __device__ __forceinline__ int prev_br(int q) const { return (int)((pbr[WIDE ? (q >> 5) : 0] >> (q & 31)) & 1u); }
-  __device__ __forceinline__ void set(int q, int rho)
-  {
-    cbl[WIDE ? (q >> 5) : 0] |= (uint32_t)((rho >> 1) & 1) << (q & 31);
-    cbr[WIDE ? (q >> 5) : 0] |= (uint32_t)((rho >> 3) & 1) << (q & 31);
-  }
-  __device__ __forceinline__ void next_row()
-  {
-#pragma unroll
-    for(int i = 0; i < (WIDE ? 16 : 1); ++i)
-    {
-      pbl[i] = cbl[i];
-      pbr[i] = cbr[i];
-      cbl[i] = cbr[i] = 0;
-    }
-  }
-};
-
-#define VLCF_SKIP(v, n) do { (v).tmp >>= (n); (v).bits -= (n); } while(0)
-template <bool WIDE>
-__global__ void __launch_bounds__(128)
-    k_ht_decode_vlc(const HtBlockDesc* __restrict__ blocks, const uint8_t* __restrict__ bytes, uint32_t* __restrict__ recs,
-                    HtBlockOut* __restrict__ status, uint32_t nblocks)
-{
-  __shared__ uint16_t tbl0[1024], tbl1[1024];
-  for(int i = threadIdx.x; i < 1024; i += blockDim.x)
-  {
-    tbl0[i] = HT_DEC_VLC0[i];
-    tbl1[i] = HT_DEC_VLC1[i];
-  }
-  __syncthreads();
-  const uint32_t bidx = blockIdx.x * blockDim.x + threadIdx.x;
-  if(bidx >= nblocks)
-    return;
-  const HtBlockDesc B = blocks[bidx];
-  const int w = B.w, h = B.h, nq = (w + 1) >> 1;
-  const uint32_t lcup = B.length;
-  const uint8_t* data = bytes + B.slot_off;
-  HtBlockOut st;
-  st.ms_len = 0; st.mel_len = 0; st.vlc_len = 0; st.total = 0;
-  int scup = 0;
-  if(lcup >= 2)
-  {
-    scup = ((int)__ldg(data + lcup - 1) << 4) + (int)(__ldg(data + lcup - 2) & 0xF);
-    if(scup < 2 || scup > (int)lcup || scup > 4079 || B.mmsbs > 29)
-      st.total = 2; /* malformed */
-  }
-  else
-    st.total = lcup == 0 ? 1 : 2; /* 1: empty block (all zero), 2: malformed */
-  if(st.total)
-  {
-    status[bidx] = st;
-    return;
-  }
-  st.ms_len = lcup - (uint32_t)scup;
-
-  MelFast mel;
-  mel.d = data + lcup - scup;
-  mel.size = scup - 1;
-  mel.pos = mel.bits = mel.unstuff = mel.k = mel.run = mel.have = 0;
-  mel.tmp = 0;
-  melf_init(mel);
-  VlcFast vlc;
-  vlc.d = data;
-  vlc.pos = (int)lcup - 3;
-  vlc.lo = (int)lcup - scup;
-  {
-    const uint32_t d = __ldg(data + lcup - 2);
-    vlc.tmp = d >> 4;
-    vlc.bits = 4 - (((vlc.tmp & 7) == 7) ? 1 : 0);
-    vlc.unstuff = (d | 0xF) > 0x8F;
-  }
-  vlcf_init(vlc);
-  uint32_t* rec = recs + B.rec_off;
-  SigRows<WIDE> sig;
-  sig.clear();
-
-  for(int y = 0; y < h; y += 2)
-  {
-    const uint16_t* tbl = y ? tbl1 : tbl0;
-    int rho_left = 0;
-    for(int q0 = 0; q0 < nq; q0 += 2)
-    {
-      vlcf_fill32(vlc);
-      const bool has1 = q0 + 1 < nq;
-      /* ---- CxtVLC of the two quads ---- */
-      int cq0, cq1 = 0;
-      if(y == 0)
-        cq0 = (rho_left >> 1) | (rho_left & 1);
-      else
-        cq0 = ((q0 > 0 ? sig.prev_br(q0 - 1) : 0) | sig.prev_bl(q0)) | ((rho_left & 0xC) ? 2 : 0) |
-              ((sig.prev_br(q0) | (has1 ? sig.prev_bl(q0 + 1) : 0)) << 2);
-      uint32_t t0 = tbl[(cq0 << 7) | (((uint32_t)vlc.tmp) & 0x7F)];
-      if(cq0 == 0 && !melf_symbol(mel))
-        t0 = 0;
-      VLCF_SKIP(vlc, (int)(t0 >> 13));
-      const int rho0 = t0 & 0xF;
-      sig.set(q0, rho0);
-      uint32_t t1 = 0;
-      int rho1 = 0;
-      if(has1)
-      {
-        if(y == 0)
-          cq1 = (rho0 >> 1) | (rho0 & 1);
-        else
-          cq1 = (sig.prev_br(q0) | sig.prev_bl(q0 + 1)) | ((rho0 & 0xC) ? 2 : 0) |
-                ((sig.prev_br(q0 + 1) | (q0 + 2 < nq ? sig.prev_bl(q0 + 2) : 0)) << 2);
-        t1 = tbl[(cq1 << 7) | (((uint32_t)vlc.tmp) & 0x7F)];
-        if(cq1 == 0 && !melf_symbol(mel))
-          t1 = 0;
-        VLCF_SKIP(vlc, (int)(t1 >> 13));
-        rho1 = t1 & 0xF;
-        sig.set(q0 + 1, rho1);
-        rho_left = rho1;
-      }
-      else
-        rho_left = rho0;
-      /* ---- UVLC (T.814 7.3.6) ---- */
-      const int uoff0 = (t0 >> 12) & 1, uoff1 = (t1 >> 12) & 1;
-      int u0 = 0, u1 = 0;
-      if(uoff0 | uoff1)
-      {
-        int len;
-        if(y == 0 && uoff0 && uoff1)
-        {
-          if(melf_symbol(mel))
-          {
-            const int p0 = uvlc_prefix(((uint32_t)vlc.tmp), len);
-            VLCF_SKIP(vlc, len);
-            const int p1 = uvlc_prefix(((uint32_t)vlc.tmp), len);
-            VLCF_SKIP(vlc, len);
-            const int l0 = uvlc_suflen(p0), l1 = uvlc_suflen(p1);
-            u0 = 2 + p0 + (int)(((uint32_t)vlc.tmp) & ((1u << l0) - 1u));
-            VLCF_SKIP(vlc, l0);
-            u1 = 2 + p1 + (int)(((uint32_t)vlc.tmp) & ((1u << l1) - 1u));
-            VLCF_SKIP(vlc, l1);
-          }
-          else
-          {
-            const int p0 = uvlc_prefix(((uint32_t)vlc.tmp), len);
-            VLCF_SKIP(vlc, len);
-            if(p0 > 2)
-            {
-              u1 = 1 + (int)(((uint32_t)vlc.tmp) & 1u);
-              VLCF_SKIP(vlc, 1);
-              const int l0 = uvlc_suflen(p0);
-              u0 = p0 + (int)(((uint32_t)vlc.tmp) & ((1u << l0) - 1u));
-              VLCF_SKIP(vlc, l0);
-            }
-            else
-            {
-              const int p1 = uvlc_prefix(((uint32_t)vlc.tmp), len);
-              VLCF_SKIP(vlc, len);
-              const int l1 = uvlc_suflen(p1);
-              u0 = p0;
-              u1 = p1 + (int)(((uint32_t)vlc.tmp) & ((1u << l1) - 1u));
-              VLCF_SKIP(vlc, l1);
-            }
-          }
-        }
-        else
-        {
-          int pf0 = 0, pf1 = 0;
-          if(uoff0)
-          {
-            pf0 = uvlc_prefix(((uint32_t)vlc.tmp), len);
-            VLCF_SKIP(vlc, len);
-          }
-          if(uoff1)
-          {
-            pf1 = uvlc_prefix(((uint32_t)vlc.tmp), len);
-            VLCF_SKIP(vlc, len);
-          }
-          if(uoff0)
-          {
-            const int l = uvlc_suflen(pf0);
-            u0 = pf0 + (int)(((uint32_t)vlc.tmp) & ((1u << l) - 1u));
-            VLCF_SKIP(vlc, l);
-          }
-          if(uoff1)
-          {
-            const int l = uvlc_suflen(pf1);
-            u1 = pf1 + (int)(((uint32_t)vlc.tmp) & ((1u << l) - 1u));
-            VLCF_SKIP(vlc, l);
-          }
-        }
-      }
-      rec[(size_t)q0 * 32] = (t0 & 0xFFFu) | ((uint32_t)u0 << 12); /* rho | e_k<<4 | e_1<<8 | u<<12 */
-      if(has1)
-        rec[(size_t)(q0 + 1) * 32] = (t1 & 0xFFFu) | ((uint32_t)u1 << 12);
-    }
-    rec += (size_t)nq * 32; /* records of 32 consecutive blocks are interleaved word by word */
-    sig.next_row();
-  }
-  status[bidx] = st;
-}
-
 /* ---------------------------------------------------------------------------------------------
- * Phase A, fast path (blocks at most 64 samples wide): the same parse, arranged so that a quad pair
- * costs one refill check, two CxtVLC look-ups and ONE U-VLC look-up instead of a tree of branches:
+ * The parse is arranged so that a quad pair costs one refill check, two CxtVLC look-ups and ONE
+ * U-VLC look-up instead of a tree of branches:
  *  - uvlc[mode * 64 + next 6 bits] holds, for the pair's two u-offset flags (mode 0..3) and for the
  *    first row's "both flags set, MEL said 0" rule (mode 4, T.814 7.3.6 / ojph_block_decoder32.cpp
  *    L966-1010), the bits the two prefixes take, the two suffix lengths and the two base values;
  *    the table is built in shared memory at kernel start from the prefix code itself;
- *  - the neighbourhood bit of a quad's context is one shift of a per-row mask (A = bl | br << 1).
- * The serial chain per quad is what bounds this phase; this halves it.
+ *  - the neighbourhood bit of a quad's context is one shift of a 64-bit mask of the row above
+ *    (A = bl | br << 1).  Blocks at most 64 samples wide (32 quads, WIDE = false) keep the row's
+ *    significance in one register word per side and build A once per row; wider ones (up to 1024
+ *    samples, 512 quads) keep 16 words per side and rebuild A every 32 quads.
+ * The serial chain per quad is what bounds this phase; this halves it against a branchy parse.
  * ------------------------------------------------------------------------------------------- */
 __device__ __forceinline__ uint32_t uvlc_entry(int mode, uint32_t bits)
 { /* plen[2:0] | l0[5:3] | l1[8:6] | p0[11:9] | p1[14:12] */
@@ -576,9 +261,10 @@ __device__ __forceinline__ uint32_t uvlc_entry(int mode, uint32_t bits)
   return (uint32_t)plen | ((uint32_t)l0 << 3) | ((uint32_t)l1 << 6) | ((uint32_t)p0 << 9) | ((uint32_t)p1 << 12);
 }
 
+template <bool WIDE>
 __global__ void __launch_bounds__(32)
-    k_ht_decode_vlc_fast(const HtBlockDesc* __restrict__ blocks, const uint8_t* __restrict__ bytes, uint32_t* __restrict__ recs,
-                         HtBlockOut* __restrict__ status, uint32_t nblocks)
+    k_ht_decode_vlc(const HtBlockDesc* __restrict__ blocks, const uint8_t* __restrict__ bytes, uint32_t* __restrict__ recs,
+                    HtBlockOut* __restrict__ status, uint32_t nblocks)
 {
   __shared__ uint16_t tbl0[1024], tbl1[1024], uvlc[5 * 64];
   for(int i = threadIdx.x; i < 1024; i += blockDim.x)
@@ -632,22 +318,35 @@ __global__ void __launch_bounds__(32)
   }
   vlcf_init(vlc);
   uint32_t* rec = recs + B.rec_off;
-  uint32_t pbl = 0, pbr = 0; /* significance of the row above's bottom-left / bottom-right samples, one bit per quad */
+  /* significance of the bottom-left / bottom-right samples of the row above (p) and of this row (c), one bit per quad,
+     32 quads per word */
+  constexpr int NW = WIDE ? 16 : 1;
+  const int nw = WIDE ? (nq + 31) >> 5 : 1;
+  uint32_t pbl[NW] = {}, pbr[NW] = {};
+  auto above = [&](int k) { /* bit j: something significant above-left or above quad 32 k + j (j up to 32) */
+    uint64_t a = (uint64_t)pbl[k] | ((uint64_t)pbr[k] << 1);
+    if constexpr(WIDE)
+      a |= (k > 0 ? pbr[k - 1] >> 31 : 0u) | (k + 1 < NW ? (uint64_t)pbl[k + 1] << 32 : 0ull);
+    return a;
+  };
 
   for(int y = 0; y < h; y += 2)
   {
     const uint16_t* tbl = y ? tbl1 : tbl0;
-    const uint64_t A = (uint64_t)pbl | ((uint64_t)pbr << 1); /* bit q: something significant above-left or above quad q (q up to 32) */
-    uint32_t cbl = 0, cbr = 0;
+    uint64_t A = above(0);
+    uint32_t cbl[NW] = {}, cbr[NW] = {};
     int rho_left = 0;
     for(int q0 = 0; q0 < nq; q0 += 2)
     {
+      const int k = WIDE ? q0 >> 5 : 0, qa = WIDE ? q0 & 31 : q0; /* the word holding quads q0, q0 + 1 and q0's bit in A */
+      if(WIDE && qa == 0 && q0 > 0)
+        A = above(k);
       vlcf_fill32(vlc);
       const bool has1 = q0 + 1 < nq;
       uint64_t tmp = vlc.tmp;
       /* ---- CxtVLC of the two quads ---- */
       const int cq0 = y == 0 ? ((rho_left >> 1) | (rho_left & 1))
-                             : (int)(((A >> q0) & 1u) | ((rho_left & 0xC) ? 2u : 0u) | (((A >> (q0 + 1)) & 1u) << 2));
+                             : (int)(((A >> qa) & 1u) | ((rho_left & 0xC) ? 2u : 0u) | (((A >> (qa + 1)) & 1u) << 2));
       uint32_t t0 = tbl[(cq0 << 7) | ((uint32_t)tmp & 0x7F)];
       if(cq0 == 0 && !melf_symbol(mel))
         t0 = 0;
@@ -659,7 +358,7 @@ __global__ void __launch_bounds__(32)
       if(has1)
       {
         const int cq1 = y == 0 ? ((rho0 >> 1) | (rho0 & 1))
-                               : (int)(((A >> (q0 + 1)) & 1u) | ((rho0 & 0xC) ? 2u : 0u) | (((A >> (q0 + 2)) & 1u) << 2));
+                               : (int)(((A >> (qa + 1)) & 1u) | ((rho0 & 0xC) ? 2u : 0u) | (((A >> (qa + 2)) & 1u) << 2));
         t1 = tbl[(cq1 << 7) | ((uint32_t)tmp & 0x7F)];
         if(cq1 == 0 && !melf_symbol(mel))
           t1 = 0;
@@ -668,8 +367,8 @@ __global__ void __launch_bounds__(32)
         rho1 = t1 & 0xF;
       }
       rho_left = has1 ? rho1 : rho0;
-      cbl |= ((uint32_t)((rho0 >> 1) & 1) << q0) | ((uint32_t)((rho1 >> 1) & 1) << (q0 + 1));
-      cbr |= ((uint32_t)((rho0 >> 3) & 1) << q0) | ((uint32_t)((rho1 >> 3) & 1) << (q0 + 1));
+      cbl[k] |= ((uint32_t)((rho0 >> 1) & 1) << qa) | ((uint32_t)((rho1 >> 1) & 1) << (qa + 1));
+      cbr[k] |= ((uint32_t)((rho0 >> 3) & 1) << qa) | ((uint32_t)((rho1 >> 3) & 1) << (qa + 1));
       /* ---- U-VLC of the pair: one look-up ---- */
       int u0 = 0, u1 = 0;
       const int uo = (int)((t0 >> 12) & 1u) | (int)(((t1 >> 12) & 1u) << 1);
@@ -703,8 +402,11 @@ __global__ void __launch_bounds__(32)
         rec[(size_t)(q0 + 1) * 32] = (t1 & 0xFFFu) | ((uint32_t)u1 << 12);
     }
     rec += (size_t)nq * 32; /* records of 32 consecutive blocks are interleaved word by word */
-    pbl = cbl;
-    pbr = cbr;
+    for(int i = 0; i < nw; ++i)
+    {
+      pbl[i] = cbl[i];
+      pbr[i] = cbr[i];
+    }
   }
   status[bidx] = st;
 }
@@ -1260,10 +962,8 @@ void b2k_launch_ht_decode_vlc(const HtBlockDesc* d_blocks, const uint8_t* d_byte
      SMs as possible instead of packing 4 warps onto one */
   if(max_w > 64)
     k_ht_decode_vlc<true><<<(nblocks + 31) / 32, 32, 0, st>>>(d_blocks, d_bytes, d_recs, d_status, nblocks);
-  else if(getenv("B2K_VLC_GENERIC")) /* the branchy reference formulation, kept for A/B runs */
-    k_ht_decode_vlc<false><<<(nblocks + 31) / 32, 32, 0, st>>>(d_blocks, d_bytes, d_recs, d_status, nblocks);
   else
-    k_ht_decode_vlc_fast<<<(nblocks + 31) / 32, 32, 0, st>>>(d_blocks, d_bytes, d_recs, d_status, nblocks);
+    k_ht_decode_vlc<false><<<(nblocks + 31) / 32, 32, 0, st>>>(d_blocks, d_bytes, d_recs, d_status, nblocks);
   b2k_count_launch();
 }
 

@@ -518,54 +518,56 @@ def test_refinement_passes_of_foreign_streams(engine, case):
 def test_corrupt_streams_are_rejected_or_decoded_never_fatal(engine):
     """Damaged block tables / byte arenas (flipped bytes, garbage Scup, wrong lengths, impossible bit-plane
     counts, bogus refinement segments): b2k_decode either decodes or reports rejected blocks (-2) or a bad
-    table (-1); it never faults, and the engine decodes a clean stream right afterwards.  (Run under
-    compute-sanitizer memcheck in profiles/r01g_memcheck.txt.)"""
+    table (-1); it never faults, and the engine decodes a clean stream right afterwards.  Blocks wider than
+    64 samples go through the wide instantiation of the VLC parse (k_ht_decode_vlc<true>), so damaged bytes
+    reach both.  (The 64x64 case was run under compute-sanitizer memcheck in profiles/r01g_memcheck.txt.)"""
     w, h = 256, 192
-    cp = G.make_coding(w, h, 3, 12, numres=4)
     planes = P.synthetic_image(w, h, 3, 12, seed=5)
-    res = engine.encode(cp, planes)
-    blocks, data = res.blocks.copy(), res.bytes.copy()
-    res.free()
-    rng = np.random.default_rng(99)
-    out = [np.zeros_like(p) for p in planes]
-    outcomes = {"ok": 0, "rejected": 0, "bad_table": 0}
-    coded = np.flatnonzero(blocks["length"] > 0)
-    for trial in range(40):
-        b, d = blocks.copy(), data.copy()
-        kind = trial % 8
-        if kind == 0:                                   # random byte flips all over the arena
-            idx = rng.integers(0, len(d), 200)
-            d[idx] ^= rng.integers(1, 256, 200).astype(np.uint8)
-        elif kind == 1:                                 # garbage Scup (last two bytes of a block)
-            for i in rng.choice(coded, 20):
-                e = int(b[i]["offset"]) + int(b[i]["length"])
-                d[e - 1], d[e - 2] = rng.integers(0, 256), rng.integers(0, 256)
-        elif kind == 2:                                 # truncated cleanup segments
-            for i in rng.choice(coded, 20):
-                b[i]["length"] = max(1, int(b[i]["length"]) // int(rng.integers(2, 6)))
-        elif kind == 3:                                 # too many bit planes for the exponents in the stream
-            for i in rng.choice(coded, 20):
-                b[i]["numbps"] = min(int(b[i]["kmax"]), int(b[i]["numbps"]) + int(rng.integers(1, 6)))
-        elif kind == 4:                                 # refinement passes pointing into the neighbour's bytes
-            for i in rng.choice(coded, 20):
-                b[i]["numpasses"], b[i]["length2"], b[i]["numbps"] = 3, min(64, len(d) - int(b[i]["offset"]) - int(b[i]["length"])), 3
-        elif kind == 5:                                 # offsets past the arena
-            b[rng.choice(coded)]["offset"] = len(d) + 1000
-        elif kind == 6:                                 # all zero bytes
-            d[:] = 0
-        else:                                           # all ones
-            d[:] = 0xFF
-        try:
-            engine.decode(cp, b, d, out)
-            outcomes["ok"] += 1
-        except G.EngineError as e:
-            msg = str(e)
-            assert "rejected" in msg or "exceed" in msg or "-1" in msg or "-2" in msg, msg
-            outcomes["rejected" if "rejected" in msg else "bad_table"] += 1
-    assert outcomes["rejected"] > 0 and outcomes["bad_table"] > 0
-    engine.decode(cp, blocks, data, out)               # still healthy
-    for a, s in zip(out, planes):
-        assert np.array_equal(a, s)
+    for cblk in ((64, 64), (1024, 4), (128, 32)):
+        cp = G.make_coding(w, h, 3, 12, numres=4, cblk=cblk)
+        res = engine.encode(cp, planes)
+        blocks, data = res.blocks.copy(), res.bytes.copy()
+        res.free()
+        rng = np.random.default_rng(99)
+        out = [np.zeros_like(p) for p in planes]
+        outcomes = {"ok": 0, "rejected": 0, "bad_table": 0}
+        coded = np.flatnonzero(blocks["length"] > 0)
+        for trial in range(40):
+            b, d = blocks.copy(), data.copy()
+            kind = trial % 8
+            if kind == 0:                                   # random byte flips all over the arena
+                idx = rng.integers(0, len(d), 200)
+                d[idx] ^= rng.integers(1, 256, 200).astype(np.uint8)
+            elif kind == 1:                                 # garbage Scup (last two bytes of a block)
+                for i in rng.choice(coded, 20):
+                    e = int(b[i]["offset"]) + int(b[i]["length"])
+                    d[e - 1], d[e - 2] = rng.integers(0, 256), rng.integers(0, 256)
+            elif kind == 2:                                 # truncated cleanup segments
+                for i in rng.choice(coded, 20):
+                    b[i]["length"] = max(1, int(b[i]["length"]) // int(rng.integers(2, 6)))
+            elif kind == 3:                                 # too many bit planes for the exponents in the stream
+                for i in rng.choice(coded, 20):
+                    b[i]["numbps"] = min(int(b[i]["kmax"]), int(b[i]["numbps"]) + int(rng.integers(1, 6)))
+            elif kind == 4:                                 # refinement passes pointing into the neighbour's bytes
+                for i in rng.choice(coded, 20):
+                    b[i]["numpasses"], b[i]["length2"], b[i]["numbps"] = 3, min(64, len(d) - int(b[i]["offset"]) - int(b[i]["length"])), 3
+            elif kind == 5:                                 # offsets past the arena
+                b[rng.choice(coded)]["offset"] = len(d) + 1000
+            elif kind == 6:                                 # all zero bytes
+                d[:] = 0
+            else:                                           # all ones
+                d[:] = 0xFF
+            try:
+                engine.decode(cp, b, d, out)
+                outcomes["ok"] += 1
+            except G.EngineError as e:
+                msg = str(e)
+                assert "rejected" in msg or "exceed" in msg or "-1" in msg or "-2" in msg, (cblk, msg)
+                outcomes["rejected" if "rejected" in msg else "bad_table"] += 1
+        assert outcomes["rejected"] > 0 and outcomes["bad_table"] > 0, (cblk, outcomes)
+        engine.decode(cp, blocks, data, out)               # still healthy
+        for a, s in zip(out, planes):
+            assert np.array_equal(a, s), cblk
 
 
 @pytest.mark.parametrize("sgnd", [False, True])
